@@ -40,6 +40,16 @@ sys.path.insert(0, str(ROOT / "tests"))
 WORKLOAD = "cone_450x375_d64_batch256"
 PAIRS_PER_STEP = 256
 METRIC = "disparity-maps/sec (450x375x64)"
+DUMP_BYTES = 60_000_000     # --dump-outputs stays below 64 MB
+
+
+def dump_outputs(out_dir: str, disp: np.ndarray) -> None:
+    """Writes the [n][H][W] float32 maps of the last timed step to out_dir/disparity.npy: all of them when they fit in
+    DUMP_BYTES, else the pairs numpy.random.default_rng(0) picks (sorted), the same ones on every run of a workload."""
+    n = disp.shape[0]
+    k = max(1, min(n, DUMP_BYTES // disp[0].nbytes))
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    np.save(Path(out_dir) / "disparity.npy", np.ascontiguousarray(disp[idx], dtype=np.float32))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -324,6 +334,8 @@ def run_gpu_arm(args):
     for s0 in range(min(seeds, n)):
         ok = ok and bool((hd[s0::seeds].view(np.uint32) == hd[s0].view(np.uint32)[None]).all())
     okd = bool(np.array_equal(dd.view(np.uint32), hd.view(np.uint32)))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dd)
     flag = torch.tensor([int(ok and okd)], dtype=torch.int32, device=dev)
     if world > 1:
         dist.all_reduce(flag, op=dist.ReduceOp.MIN)
@@ -473,6 +485,8 @@ def run_sharded_arm(args, eng, dev, rank, world, n, w, h, D, wl_name, np_left, n
     if rank == 0:
         golden = _golden_final_sha(args.workload)
         out = d_out.cpu().numpy()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, out)
         check["golden"] = all(T.sha(out[i]) == sha for i, sha in golden.items())
         bad = [int(i) for i in range(total) if not np.array_equal(out[i].view(np.uint32), out[i % seeds].view(np.uint32))]
         check["copies_equal"] = not bad
@@ -522,7 +536,14 @@ def main():
                     help="BASELINE configs[4] form: one batch of pairs x gpus owned by rank 0, NCCL scatter -> Match -> NCCL gather")
     ap.add_argument("--workload", default="cone", choices=["cone", "kitti", "1080p"],
                     help="cone = BASELINE configs[1] (the contract metric); kitti / 1080p = configs[2] / configs[3] (extra lines)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the disparity maps of the last timed (device-resident) step to "
+                         "DIR/disparity.npy, float32 [k][H][W]: the whole batch, or a fixed sample of it below 64 MB")
     args = ap.parse_args()
+    if args.dump_outputs:
+        if args.impl == "reference":
+            ap.error("--dump-outputs writes the GPU path's maps; the reference arm keeps none")
+        Path(args.dump_outputs).mkdir(parents=True, exist_ok=True)
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_gpu_arm(args)

@@ -74,7 +74,9 @@ def build_oracle(force: bool = False) -> None:
     if force or not target.exists() or any(s.stat().st_mtime > target.stat().st_mtime for s in srcs):
         subprocess.run(["make", "-C", str(ORACLE_DIR), "oracle"], check=True, capture_output=True)
     ref = ORACLE_DIR / "_ref" / "libadcensus_ref.so"
-    if (REFERENCE_ROOT / "AD-Census").is_dir():
+    # os.access, not Path.is_dir: a user who may not enter the reference's parent directory gets
+    # False here instead of a PermissionError, and keeps the committed goldens as the only pin
+    if os.access(REFERENCE_ROOT / "AD-Census", os.R_OK | os.X_OK):
         if force or not ref.exists() or (ORACLE_DIR / "ref_harness.cpp").stat().st_mtime > ref.stat().st_mtime:
             subprocess.run(["make", "-C", str(ORACLE_DIR), "ref"], check=True, capture_output=True)
 
