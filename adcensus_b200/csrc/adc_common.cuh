@@ -158,3 +158,8 @@ void adc_launch_cloud(const AdcParams& P, const AdcWave& w1, const float* d_disp
                       cudaStream_t st, unsigned long long* launches);
 int adc_launch_median(const AdcParams& P, const AdcWave& w, const float* in, float* out, cudaStream_t st,
                       unsigned long long* launches);
+// Dynamic shared memory one launch of the kernel needs at these sizes, and in *cap the most its function attribute
+// grants (adc_create refuses sizes for which need > cap)
+size_t adc_cost_smem(const AdcDims& dm, size_t* cap);
+size_t adc_scanline_smem(const AdcDims& dm, size_t* cap);
+size_t adc_voting_smem(const AdcDims& dm, size_t* cap);

@@ -11,7 +11,7 @@
 
 static_assert(sizeof(ADCensusOption) == sizeof(adc_option), "option block must be byte-compatible with the C ABI");
 
-ADCensusStereo::ADCensusStereo() : engine_(nullptr), width_(0), height_(0), is_initialized_(false) {}
+ADCensusStereo::ADCensusStereo() : engine_(nullptr), width_(0), height_(0), max_disparity_range_(0), is_initialized_(false) {}
 
 ADCensusStereo::~ADCensusStereo() {
     Release();
@@ -24,9 +24,15 @@ void ADCensusStereo::Release() {
 }
 
 bool ADCensusStereo::Initialize(const sint32& width, const sint32& height, const ADCensusOption& option) {
+    return Initialize(width, height, option, 0);
+}
+
+bool ADCensusStereo::Initialize(const sint32& width, const sint32& height, const ADCensusOption& option,
+                                sint32 max_disparity_range) {
     width_ = width;
     height_ = height;
     option_ = option;
+    max_disparity_range_ = max_disparity_range;
     Release();  // the reference leaks on a second Initialize; here the old engine is freed
     is_initialized_ = false;
     adc_option raw;
@@ -34,6 +40,7 @@ bool ADCensusStereo::Initialize(const sint32& width, const sint32& height, const
     adc_config cfg;
     std::memset(&cfg, 0, sizeof(cfg));
     if (const char* dev = std::getenv("ADC_B200_DEVICE")) cfg.device = std::atoi(dev);
+    cfg.max_disparity_range = max_disparity_range;
     if (adc_create(width, height, &raw, &cfg, &engine_) != ADC_OK) {
         engine_ = nullptr;
         return false;
@@ -64,7 +71,7 @@ bool ADCensusStereo::Match(const uint8* img_left, const uint8* img_right, float3
 bool ADCensusStereo::Reset(const uint32& width, const uint32& height, const ADCensusOption& option) {
     Release();
     is_initialized_ = false;
-    return Initialize(static_cast<sint32>(width), static_cast<sint32>(height), option);
+    return Initialize(static_cast<sint32>(width), static_cast<sint32>(height), option, max_disparity_range_);
 }
 
 bool ADCensusStereo::MatchBatch(sint32 n, const uint8* left, const uint8* right, float32* disp) {

@@ -27,6 +27,8 @@ static_assert(sizeof(adc_option) == 60, "adc_option must match the reference's A
 static_assert(offsetof(adc_option, so_p1) == 32 && offsetof(adc_option, irv_th) == 48 &&
               offsetof(adc_option, do_lr_check) == 56 && offsetof(adc_option, do_discontinuity_adjustment) == 58,
               "adc_option field offsets must match adcensus_types.h:45-75");
+static_assert(sizeof(adc_config) == 64 && offsetof(adc_config, max_disparity_range) == 16,
+              "adc_config layout is part of the ABI: 64 bytes, max_disparity_range at offset 16");
 
 namespace {
 
@@ -303,7 +305,8 @@ int enqueue_pipeline(adc_engine* e, Lane& ln, int nS, int last_stage, cudaEvent_
         const float* src = (ps % 2 == 0) ? A : B;
         float* dst = (ps % 2 == 0) ? B : A;
         if (adc_launch_scanline(P, w, src, dst, dirs[ps][0], dirs[ps][1], st, L))
-            return fail(ADC_ERR_UNSUPPORTED, "disparity range %d exceeds the scanline kernel's limit of 256", P.dm.D);
+            return fail(ADC_ERR_UNSUPPORTED, "disparity range %d exceeds the scanline kernel's limit of %d", P.dm.D,
+                        ADC_MAX_DISPARITY_RANGE_WIDE);
         if (ps % 2 == 0) e->dbg_init = B; else e->dbg_aggr = A;
         if (stop(ADC_STAGE_SO1 + ps)) return launched("scanline optimisation");
     }
@@ -500,9 +503,14 @@ int adc_create(int32_t width, int32_t height, const adc_option* opt, const adc_c
     // Limits of the kernels (the reference has none; INTEGRATION.md lists them).  They are checked HERE, so that a caller
     // never sees Initialize() succeed and Match() fail for a size: whatever adc_create accepts, adc_match runs.
     const int drange = opt->max_disparity - opt->min_disparity;
+    const int limit_cfg = cfg ? cfg->max_disparity_range : 0;
+    if (limit_cfg < 0 || limit_cfg > ADC_MAX_DISPARITY_RANGE_WIDE)
+        return fail(ADC_ERR_ARG, "adc_create: max_disparity_range %d outside 0..%d", limit_cfg, ADC_MAX_DISPARITY_RANGE_WIDE);
+    const int limit = limit_cfg ? limit_cfg : ADC_MAX_DISPARITY_RANGE;
     if ((long long)width * height > (1ll << 28)) return fail(ADC_ERR_UNSUPPORTED, "adc_create: image too large (more than 2^28 pixels)");
-    if (drange > ADC_MAX_DISPARITY_RANGE)
-        return fail(ADC_ERR_UNSUPPORTED, "adc_create: disparity range %d > %d is not supported (scanline kernel: 8 disparities per lane)", drange, ADC_MAX_DISPARITY_RANGE);
+    if (drange > limit)
+        return fail(ADC_ERR_UNSUPPORTED, "adc_create: disparity range %d > %d is not supported by this engine (adc_config.max_disparity_range "
+                    "raises the limit up to %d)", drange, limit, ADC_MAX_DISPARITY_RANGE_WIDE);
     if (height > ADC_MAX_HEIGHT)
         return fail(ADC_ERR_UNSUPPORTED, "adc_create: image height %d > %d is not supported (in-place median: one CTA per image)", height, ADC_MAX_HEIGHT);
     if (width > ADC_MAX_WIDTH || width + drange > ADC_MAX_WIDTH)
@@ -511,7 +519,22 @@ int adc_create(int32_t width, int32_t height, const adc_option* opt, const adc_c
     adc_engine* e = new adc_engine();
     e->W = width; e->H = height; e->opt = *opt;
     if (cfg) e->cfg = *cfg;
+    e->cfg.max_disparity_range = limit;
     build_params(e);
+    // kernels whose shared memory grows with the sizes: a launch that could not get its shared memory must fail here
+    {
+        struct { const char* name; size_t (*need)(const AdcDims&, size_t*); } smem[] = {
+            {"cost volume", adc_cost_smem}, {"scanline", adc_scanline_smem}, {"region voting", adc_voting_smem}};
+        for (const auto& k : smem) {
+            size_t cap = 0;
+            const size_t need = k.need(e->P.dm, &cap);
+            if (need > cap) {
+                delete e;
+                return fail(ADC_ERR_UNSUPPORTED, "adc_create: the %s kernel needs %zu bytes of shared memory at %dx%d, disparity "
+                            "range %d (at most %zu)", k.name, need, width, height, drange, cap);
+            }
+        }
+    }
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         delete e;

@@ -191,10 +191,21 @@ k_cost_volume(AdcDims dm, int gpc, int nseg, int Lx, int rpc, const unsigned* __
     }
 }
 
+#define CV_SMEM_ATTR (96 * 1024)
+static int cv_nseg(int W) { return (W + CV_SEG_COLS - 1) / CV_SEG_COLS; }
+static int cv_seg_len(int W) { const int nseg = cv_nseg(W); return (((W + nseg - 1) / nseg) + 3) & ~3; }   // a multiple of 4
+static size_t cv_smem_bytes(int Lx, int D) { return (size_t)(64 * 32 + 766 * CV_AD_REP) * 4 + (size_t)3 * cv_row_len(Lx, D) * 4 + (size_t)3 * Lx * 4; }
+
+// at Lx = CV_SEG_COLS and D = 512: 85,680 bytes
+size_t adc_cost_smem(const AdcDims& dm, size_t* cap) {
+    *cap = CV_SMEM_ATTR;
+    return cv_smem_bytes(cv_seg_len(dm.W), dm.D);
+}
+
 void adc_launch_cost(const AdcParams& P, const AdcWave& w, float* vol, cudaStream_t st, unsigned long long* launches) {
     const int Q = P.dm.Dp / 4;
-    const int nseg = (P.dm.W + CV_SEG_COLS - 1) / CV_SEG_COLS;
-    const int Lx = (((P.dm.W + nseg - 1) / nseg) + 3) & ~3;                // columns per segment, a multiple of 4
+    const int nseg = cv_nseg(P.dm.W);
+    const int Lx = cv_seg_len(P.dm.W);                                     // columns per segment
     const int groups = Lx / 4;
     int gmax = 512 / Q;                             // pixel groups in flight per CTA
     if (gmax > 32) gmax = 32;
@@ -202,11 +213,11 @@ void adc_launch_cost(const AdcParams& P, const AdcWave& w, float* vol, cudaStrea
     const int trips = (groups + gmax - 1) / gmax;
     const int gpc = (groups + trips - 1) / trips;   // ... evened out over the trips
     const int threads = (gpc * Q + 31) / 32 * 32;
-    const size_t smem = (size_t)(64 * 32 + 766 * CV_AD_REP) * 4 + (size_t)3 * cv_row_len(Lx, P.dm.D) * 4 + (size_t)3 * Lx * 4;
+    const size_t smem = cv_smem_bytes(Lx, P.dm.D);
     static AdcOnce attr_once;
     if (adc_once_needed(attr_once)) {
-        cudaFuncSetAttribute(k_cost_volume<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-        cudaFuncSetAttribute(k_cost_volume<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+        cudaFuncSetAttribute(k_cost_volume<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, CV_SMEM_ATTR);
+        cudaFuncSetAttribute(k_cost_volume<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, CV_SMEM_ATTR);
         adc_once_done(attr_once);
     }
     const int rpc = 4;                              // rows per CTA: the 57 KB of tables are staged once per four rows

@@ -102,7 +102,7 @@ void adc_launch_outlier(const AdcParams& P, const AdcWave& w, cudaStream_t st, u
 // =============================================================================================
 #define RV_THREADS 1024
 #define RV_WARPS (RV_THREADS / 32)
-#define RV_MAXD 256
+#define RV_MAXD 256     // histogram bins of the byte-state kernel (D <= 254); the float-state kernel sizes its own
 #define RV_TILE 16
 
 // ---- ordered (raster) pixel lists of the two outlier classes: row counts -> scan -> scatter ----
@@ -256,7 +256,7 @@ template <bool USE_L1>
 __global__ void __cluster_dims__(RV_CLUSTER, 1, 1) __launch_bounds__(RV_THREADS)
 k_region_voting_global(AdcParams P, const uchar4* __restrict__ arms, float* disp_old, float* disp_new,
                        uint8_t* label, int* pend, int* counters, int* tile_stamp, int* last_eval) {
-    __shared__ int s_hist[RV_WARPS][RV_MAXD];
+    extern __shared__ int rv_hist[];   // [RV_WARPS][D]: one histogram per warp (dynamic: up to 64 KB at D = 512)
     __shared__ int s_tot[RV_WARPS];
     const AdcDims& dm = P.dm;
     const int pair = blockIdx.x / RV_CLUSTER;
@@ -276,7 +276,7 @@ k_region_voting_global(AdcParams P, const uchar4* __restrict__ arms, float* disp
     int* cnt = counters + pair * ADC_CNT;   // 0,1: list sizes   2: rounds   3: evaluations   4..6: change flags (mod 3)
     int n_list[2] = {__ldcg(cnt + 0), __ldcg(cnt + 1)};
     int rounds_total = 0, evals = 0;
-    int* hist = s_hist[wid];
+    int* hist = rv_hist + wid * D;
 
     // nothing stamped, nothing evaluated: stamp(0) >= last_eval(0) makes the first round evaluate everyone
     for (int i = gtid; i < tw * th; i += n_gthreads) __stcg(tiles + i, 0);
@@ -620,7 +620,13 @@ k_region_voting_bytes(AdcParams P, const uchar4* __restrict__ arms, const uchar2
 // Three kernels, chosen by the parameters alone (each has its parity cases in tests/test_gpu_parity.py):
 //   D <= 254 and L1 <= 127   incremental histograms, k_vote.cu (every BASELINE configuration)
 //   D <= 254, L1 > 127       byte-state pull kernel (a cross region may hold more than 65535 pixels)
-//   D = 255, 256             float-state pull kernel (the byte state codes a disparity index in one byte)
+//   D = 255 .. 512           float-state pull kernel (the byte state codes a disparity index in one byte)
+#define RV_GLOBAL_SMEM_ATTR (RV_WARPS * 512 * 4)
+size_t adc_voting_smem(const AdcDims& dm, size_t* cap) {
+    *cap = RV_GLOBAL_SMEM_ATTR;
+    return dm.D <= 254 ? 0 : (size_t)RV_WARPS * dm.D * 4;   // (the D <= 254 kernels' histograms are static / budgeted in k_vote.cu)
+}
+
 void adc_launch_voting(const AdcParams& P, const AdcWave& w, cudaStream_t st, unsigned long long* launches) {
     // disp_l = committed state (OLD), disp_t = working copy (NEW); both hold the post-outlier map here
     dim3 egrid((P.dm.N + 255) / 256, w.S);
@@ -635,8 +641,14 @@ void adc_launch_voting(const AdcParams& P, const AdcWave& w, cudaStream_t st, un
         }
         adc_launch_build_lists(P, w, st, launches);   // outlier lists = every listed pixel that is still invalid
     } else {
-        k_region_voting_global<false><<<w.S * RV_CLUSTER, RV_THREADS, 0, st>>>(P, w.arms, w.disp_l, w.disp_t, w.label, w.pend,
-                                                                               w.counters, w.tile_stamp, w.last_eval);
+        static AdcOnce attr_once;
+        if (adc_once_needed(attr_once)) {
+            cudaFuncSetAttribute(k_region_voting_global<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, RV_GLOBAL_SMEM_ATTR);
+            adc_once_done(attr_once);
+        }
+        size_t cap;
+        k_region_voting_global<false><<<w.S * RV_CLUSTER, RV_THREADS, adc_voting_smem(P.dm, &cap), st>>>(
+            P, w.arms, w.disp_l, w.disp_t, w.label, w.pend, w.counters, w.tile_stamp, w.last_eval);
         ++*launches;
     }
 }

@@ -368,16 +368,30 @@ k_scanline(AdcParams P, const float* __restrict__ src, float* __restrict__ dst,
     if (!BULK) cp_async_wait<0>();
 }
 
+#define SO_SMEM_ATTR (160 * 1024)
+// ring (+ mbarriers) of one CTA; at Dp = 512 (one line per warp, bulk ring): 68,352 bytes
+static size_t so_smem_bytes(int Dp, int LPS, bool bulk) {
+    const int slot_bytes = (Dp + so_rec_words(Dp)) * 4;
+    return (size_t)SO_WARPS * SO_PF * ((size_t)(32 / LPS) * slot_bytes + (bulk ? 8 : 0));
+}
+// lanes per line: as few as keep K = ceil(Dp / lanes) <= 8, a whole warp beyond Dp = 256 (K = 9 .. 16)
+static int so_lanes_per_line(int Dp) { return Dp <= 64 ? 8 : (Dp <= 128 ? 16 : 32); }
+
+size_t adc_scanline_smem(const AdcDims& dm, size_t* cap) {
+    *cap = SO_SMEM_ATTR;
+    const int LPS = so_lanes_per_line(dm.Dp);
+    return so_smem_bytes(dm.Dp, LPS, LPS == 32);
+}
+
 template <int K, int LPS, bool FULL, bool BULK>
 static int launch_scanline_kf(const AdcParams& P, const AdcWave& w, const float* src, float* dst, int sx, int sy,
                              cudaStream_t st) {
     constexpr int LPW = 32 / LPS;
     const int n_lines = sx ? P.dm.H : P.dm.W;
-    const int slot_bytes = (P.dm.Dp + so_rec_words(P.dm.Dp)) * 4;
-    const size_t smem = (size_t)SO_WARPS * SO_PF * ((size_t)LPW * slot_bytes + (BULK ? 8 : 0));
+    const size_t smem = so_smem_bytes(P.dm.Dp, LPS, BULK);
     static AdcOnce attr_once;
     if (adc_once_needed(attr_once)) {
-        cudaFuncSetAttribute(k_scanline<K, LPS, FULL, BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
+        cudaFuncSetAttribute(k_scanline<K, LPS, FULL, BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SO_SMEM_ATTR);
         adc_once_done(attr_once);
     }
     const int lines_per_block = SO_WARPS * LPW;
@@ -410,7 +424,7 @@ void adc_launch_so_bitrows(const AdcParams& P, const AdcWave& w, cudaStream_t st
 
 int adc_launch_scanline(const AdcParams& P, const AdcWave& w, const float* src, float* dst, int sx, int sy,
                         cudaStream_t st, unsigned long long* launches) {
-    // lanes per line: as few as keep K = ceil(Dp / lanes) <= 8 (Dp is a multiple of 4)
+    // lanes per line: see so_lanes_per_line (Dp is a multiple of 4)
     const int Dp = P.dm.Dp;
     int rc = 1;
 #define SO_GO(KK, LL) rc = launch_scanline_k<KK, LL>(P, w, src, dst, sx, sy, st)
@@ -421,7 +435,11 @@ int adc_launch_scanline(const AdcParams& P, const AdcWave& w, const float* src, 
         switch ((Dp + 15) / 16) { case 5: SO_GO(5, 16); break; case 6: SO_GO(6, 16); break; case 7: SO_GO(7, 16); break; default: SO_GO(8, 16); }
     } else if (Dp <= 256) {    // a whole warp per line
         switch ((Dp + 31) / 32) { case 5: SO_GO(5, 32); break; case 6: SO_GO(6, 32); break; case 7: SO_GO(7, 32); break; default: SO_GO(8, 32); }
-    } else return 1;           // D > 256 not supported
+    } else if (Dp <= 512) {    // a whole warp per line, 9 .. 16 disparities per lane (engines created with a wide range limit)
+        switch ((Dp + 31) / 32) { case 9: SO_GO(9, 32); break; case 10: SO_GO(10, 32); break; case 11: SO_GO(11, 32); break;
+                                  case 12: SO_GO(12, 32); break; case 13: SO_GO(13, 32); break; case 14: SO_GO(14, 32); break;
+                                  case 15: SO_GO(15, 32); break; default: SO_GO(16, 32); }
+    } else return 1;           // D > 512 not supported
 #undef SO_GO
     ++*launches;
     return rc;

@@ -47,7 +47,13 @@ assert ctypes.sizeof(ADCensusOption) == 60
 
 class _Config(ctypes.Structure):
     _fields_ = [("device", ctypes.c_int32), ("wave_pairs", ctypes.c_int32), ("lanes", ctypes.c_int32),
-                ("debug_flags", ctypes.c_int32), ("reserved", ctypes.c_int32 * 12)]
+                ("debug_flags", ctypes.c_int32), ("max_disparity_range", ctypes.c_int32), ("reserved", ctypes.c_int32 * 11)]
+
+
+assert ctypes.sizeof(_Config) == 64 and _Config.max_disparity_range.offset == 16
+
+# adc_config.max_disparity_range: 0 = MAX_DISPARITY_RANGE; an engine may raise its limit up to MAX_DISPARITY_RANGE_WIDE
+MAX_DISPARITY_RANGE, MAX_DISPARITY_RANGE_WIDE = 256, 512
 
 
 # adc_config.debug_flags (test hooks)
@@ -127,18 +133,22 @@ class Engine:
     """Thin object wrapper over adc_create/.../adc_destroy."""
 
     def __init__(self, width: int, height: int, option: ADCensusOption | None = None, device: int = 0,
-                 wave_pairs: int = 0, lanes: int = 0, debug_flags: int = 0):
+                 wave_pairs: int = 0, lanes: int = 0, debug_flags: int = 0, max_disparity_range: int = 0):
+        """max_disparity_range: the largest max_disparity - min_disparity this engine accepts; 0 = MAX_DISPARITY_RANGE,
+        at most MAX_DISPARITY_RANGE_WIDE."""
         self._L = load_library()
         self.width, self.height = int(width), int(height)
         self.option = option or ADCensusOption()
         self.D = self.option.max_disparity - self.option.min_disparity
-        cfg = _Config(device=device, wave_pairs=wave_pairs, lanes=lanes, debug_flags=debug_flags)
+        cfg = _Config(device=device, wave_pairs=wave_pairs, lanes=lanes, debug_flags=debug_flags,
+                      max_disparity_range=max_disparity_range)
         h = ctypes.c_void_p()
         _check(self._L.adc_create(self.width, self.height, ctypes.byref(self.option), ctypes.byref(cfg), ctypes.byref(h)))
         self._h = h
         got = _Config()
         self._L.adc_get_config(self._h, ctypes.byref(got))
         self.wave_pairs, self.lanes, self.device = got.wave_pairs, got.lanes, got.device
+        self.max_disparity_range = got.max_disparity_range
 
     def close(self):
         if getattr(self, "_h", None):
@@ -277,12 +287,15 @@ class ADCensusStereo:
 
     def __init__(self):
         self._engine = None
+        self._max_disparity_range = 0
         self.last_error = ""
 
-    def Initialize(self, width: int, height: int, option: ADCensusOption) -> bool:
+    def Initialize(self, width: int, height: int, option: ADCensusOption, max_disparity_range: int = 0) -> bool:
+        """max_disparity_range (extension, not in the reference): the engine's disparity range limit, see Engine."""
         self.Release()
+        self._max_disparity_range = max_disparity_range
         try:
-            self._engine = Engine(width, height, option)
+            self._engine = Engine(width, height, option, max_disparity_range=max_disparity_range)
         except (AdcError, ValueError) as e:
             self.last_error = str(e)
             self._engine = None
@@ -302,7 +315,7 @@ class ADCensusStereo:
 
     def Reset(self, width: int, height: int, option: ADCensusOption) -> bool:
         self.Release()
-        return self.Initialize(width, height, option)
+        return self.Initialize(width, height, option, self._max_disparity_range)
 
     def Release(self):
         if self._engine is not None:

@@ -37,6 +37,10 @@ public:
     bool Reset(const uint32& width, const uint32& height, const ADCensusOption& option);
 
     // ---- extensions (not in the reference) ----
+    // Initialize with this object's disparity range limit set (adc_config.max_disparity_range: 0 = the default
+    // ADC_MAX_DISPARITY_RANGE, at most ADC_MAX_DISPARITY_RANGE_WIDE); Reset keeps the limit.  The three-argument
+    // Initialize uses the default limit.
+    bool Initialize(const sint32& width, const sint32& height, const ADCensusOption& option, sint32 max_disparity_range);
     // n independent pairs in one call: left/right [n][H][W][3], disp [n][H][W] (host memory).
     bool MatchBatch(sint32 n, const uint8* left, const uint8* right, float32* disp);
     adc_engine* handle() const { return engine_; }
@@ -46,6 +50,7 @@ private:
     adc_engine* engine_;
     sint32 width_, height_;
     ADCensusOption option_;
+    sint32 max_disparity_range_;
     bool is_initialized_;
 };
 

@@ -61,7 +61,10 @@ typedef struct adc_config {
     int32_t lanes;           /* concurrent waves in flight, one stream each (default: auto) */
     int32_t debug_flags;     /* test hooks, 0 in production: force the alternate code paths that otherwise only unusual
                                 parameters reach, so that the parity tests can run every shipped kernel (ADC_DBG_*) */
-    int32_t reserved[12];    /* must be zero */
+    int32_t max_disparity_range; /* offset 16: largest max_disparity - min_disparity this engine accepts.  0 =
+                                ADC_MAX_DISPARITY_RANGE; 1 .. ADC_MAX_DISPARITY_RANGE_WIDE raise (or lower) it; anything
+                                else fails adc_create with ADC_ERR_ARG.  adc_get_config reports the resolved value. */
+    int32_t reserved[11];    /* must be zero */
 } adc_config;
 
 enum {
@@ -75,15 +78,18 @@ enum {
 void adc_default_option(adc_option* opt);
 
 /* Sizes the kernels implement; the reference has no such limits (it only rejects non-positive sizes).  A configuration
- * outside them fails at adc_create / Initialize with ADC_ERR_UNSUPPORTED -- never later, in adc_match. */
-#define ADC_MAX_DISPARITY_RANGE 256   /* max_disparity - min_disparity */
+ * outside them fails at adc_create / Initialize with ADC_ERR_UNSUPPORTED -- never later, in adc_match.
+ * The disparity range limit is per engine: ADC_MAX_DISPARITY_RANGE unless adc_config.max_disparity_range sets another
+ * value, at most ADC_MAX_DISPARITY_RANGE_WIDE (the scanline kernel keeps up to 16 disparities per lane of a warp). */
+#define ADC_MAX_DISPARITY_RANGE 256        /* max_disparity - min_disparity, default limit */
+#define ADC_MAX_DISPARITY_RANGE_WIDE 512   /* largest limit adc_config.max_disparity_range may set */
 #define ADC_MAX_HEIGHT 4096
 #define ADC_MAX_WIDTH 10000           /* also bounds width + disparity range */
 
 /* stands in for: ADCensusStereo::Initialize(width, height, option) (ADCensusStereo.h:25,
  * ADCensusStereo.cpp:21-67).  cfg may be NULL.  Fails (ADC_ERR_ARG) exactly where Initialize
- * returns false: width<=0, height<=0, max_disparity-min_disparity<=0; fails with ADC_ERR_UNSUPPORTED beyond the
- * limits above. */
+ * returns false: width<=0, height<=0, max_disparity-min_disparity<=0, and on a cfg->max_disparity_range outside
+ * 0 .. ADC_MAX_DISPARITY_RANGE_WIDE; fails with ADC_ERR_UNSUPPORTED beyond the limits above. */
 int adc_create(int32_t width, int32_t height, const adc_option* opt, const adc_config* cfg, adc_engine** out);
 
 /* stands in for: ADCensusStereo::~ADCensusStereo / Release (ADCensusStereo.cpp:15-19,312-316) */
