@@ -7,9 +7,9 @@ This package is the Python mirror of the reference's interface for that path
 ``adcensus_types.h:45-75`` and ``ADCensusStereo.h:14-95``).  There is no CPU fallback: importing
 works anywhere, but creating an engine without the CUDA library or without a GPU raises.
 """
-from .engine import (ADCensusOption, ADCensusStereo, AdcError, Engine, STAGE, TAP, lib_path,  # noqa: F401
+from .engine import (ADCensusOption, ADCensusStereo, AdcError, AuxOutputs, Engine, STAGE, TAP, lib_path,  # noqa: F401
                      load_library, Invalid_Float)
 from .build import build_library  # noqa: F401
 
-__all__ = ["ADCensusOption", "ADCensusStereo", "AdcError", "Engine", "STAGE", "TAP", "lib_path",
+__all__ = ["ADCensusOption", "ADCensusStereo", "AdcError", "AuxOutputs", "Engine", "STAGE", "TAP", "lib_path",
            "load_library", "build_library", "Invalid_Float"]

@@ -141,6 +141,21 @@ size_t adc_so_bitrow_bytes(const AdcDims& dm);
 int adc_launch_scanline(const AdcParams& P, const AdcWave& w, const float* src, float* dst, int sx, int sy,
                         cudaStream_t st, unsigned long long* launches);
 int adc_launch_wta(const AdcParams& P, const AdcWave& w, const float* vol, cudaStream_t st, unsigned long long* launches);
+// Device buffers of the side outputs of one wave ([S][N] each; NULL = not wanted).  `origin` is written in two steps: the
+// WTA kernel stores the WTA-invalid flag, adc_launch_origin ORs the code on; `lab0` keeps the outlier labels from
+// before region voting (only with `origin`).
+struct AdcAux {
+    uint8_t* origin;
+    uint8_t* lab0;
+    float* cost_best;
+    float* cost_second;
+};
+// the same WTA, also writing cost_best / cost_second / the WTA-invalid flag of the left view where aux asks for them
+int adc_launch_wta_aux(const AdcParams& P, const AdcWave& w, const float* vol, const AdcAux& aux, cudaStream_t st,
+                       unsigned long long* launches);
+// origin code of every pixel from aux.lab0, the labels after voting (w.label) and the map after the last filling step
+// (w.disp_l)
+void adc_launch_origin(const AdcParams& P, const AdcWave& w, const AdcAux& aux, cudaStream_t st, unsigned long long* launches);
 void adc_launch_outlier(const AdcParams& P, const AdcWave& w, cudaStream_t st, unsigned long long* launches);
 void adc_launch_build_lists(const AdcParams& P, const AdcWave& w, cudaStream_t st, unsigned long long* launches);
 void adc_launch_voting(const AdcParams& P, const AdcWave& w, cudaStream_t st, unsigned long long* launches);

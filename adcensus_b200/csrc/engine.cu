@@ -29,6 +29,9 @@ static_assert(offsetof(adc_option, so_p1) == 32 && offsetof(adc_option, irv_th) 
               "adc_option field offsets must match adcensus_types.h:45-75");
 static_assert(sizeof(adc_config) == 64 && offsetof(adc_config, max_disparity_range) == 16,
               "adc_config layout is part of the ABI: 64 bytes, max_disparity_range at offset 16");
+static_assert(sizeof(adc_aux_outputs) == 32 && offsetof(adc_aux_outputs, origin) == 0 &&
+              offsetof(adc_aux_outputs, cost_best) == 8 && offsetof(adc_aux_outputs, cost_second) == 16 &&
+              offsetof(adc_aux_outputs, disp_right) == 24, "adc_aux_outputs layout is part of the ABI: four pointers, 32 bytes");
 
 namespace {
 
@@ -65,6 +68,12 @@ struct Lane {
     float* const* drain_ptrs = nullptr;
     float* drain_base = nullptr;
     int drain_first = 0;
+    // side outputs, allocated by the first call that asks for them (ensure_aux)
+    void* aux_arena = nullptr;         // device scratch of the wave: origin, lab0, cost_best, cost_second, [S][N] each
+    AdcAux aux{};
+    void* aux_pin = nullptr;           // pinned staging of the four outputs (pageable callers)
+    adc_aux_outputs pin_aux{};         // ... carved: origin, cost_best, cost_second, disp_right, [S][N] each
+    adc_aux_outputs drain_aux{};       // the caller's side-output buffers of the pending copy-out (NULL members: none)
 };
 
 }  // namespace
@@ -239,7 +248,8 @@ AdcWave wave_view(const adc_engine* e, const Lane& ln, int nS) {
 // Enqueues the whole pipeline for the nS pairs whose images already sit in ln.w.bgr.  Stops after
 // `last_stage` (ADC_STAGE_MEDIAN = everything).  ev[] (optional, 6 events) are recorded at the
 // stage boundaries the reference times in Match (ADCensusStereo.cpp:81-129).
-int enqueue_pipeline(adc_engine* e, Lane& ln, int nS, int last_stage, cudaEvent_t* ev) {
+// `aux` (optional): device buffers of the side outputs this run writes besides the map; NULL = the plain pipeline.
+int enqueue_pipeline(adc_engine* e, Lane& ln, int nS, int last_stage, cudaEvent_t* ev, const AdcAux* aux = nullptr) {
     const AdcParams& P = e->P;
     const AdcWave w = wave_view(e, ln, nS);
     cudaStream_t st = ln.st;
@@ -314,7 +324,9 @@ int enqueue_pipeline(adc_engine* e, Lane& ln, int nS, int last_stage, cudaEvent_
     if (ev) CK(cudaEventRecord(ev[3], st));
 
     // ---- stage 4: left + right disparity (ADCensusStereo.cpp:108-109)
-    if (adc_launch_wta(P, w, A, st, L)) return fail(ADC_ERR_UNSUPPORTED, "WTA launch failed");
+    const bool wta_aux = aux && (aux->origin || aux->cost_best || aux->cost_second);
+    if (wta_aux ? adc_launch_wta_aux(P, w, A, *aux, st, L) : adc_launch_wta(P, w, A, st, L))
+        return fail(ADC_ERR_UNSUPPORTED, "WTA launch failed");
     if ((rc = launched("winner-takes-all"))) return rc;
     if (ev) CK(cudaEventRecord(ev[4], st));
     if (stop(ADC_STAGE_WTA)) return ADC_OK;
@@ -327,6 +339,7 @@ int enqueue_pipeline(adc_engine* e, Lane& ln, int nS, int last_stage, cudaEvent_
         CK(cudaMemsetAsync(w.label, 0, mapN, st));
         CK(cudaMemcpyAsync(w.disp_t, w.disp_l, mapN * sizeof(float), cudaMemcpyDeviceToDevice, st));
     }
+    if (aux && aux->origin) CK(cudaMemcpyAsync(aux->lab0, w.label, mapN, cudaMemcpyDeviceToDevice, st));   // voting clears labels
     if (stop(ADC_STAGE_OUTLIER)) return launched("outlier detection");
     if (e->opt.do_filling) {  // gates voting AND interpolation (ADCensusStereo.cpp:183)
         CK(cudaMemsetAsync(w.counters, 0, (size_t)nS * ADC_CNT * sizeof(int), st));
@@ -343,6 +356,7 @@ int enqueue_pipeline(adc_engine* e, Lane& ln, int nS, int last_stage, cudaEvent_
         e->dbg_stage = last_stage;
         return launched("refinement");
     }
+    if (aux && aux->origin) adc_launch_origin(P, w, *aux, st, L);
     if (e->opt.do_discontinuity_adjustment) adc_launch_discontinuity(P, w, A, st, L);
     if (stop(ADC_STAGE_DISC)) return launched("discontinuity adjustment");
     // median: disp_l -> disp_t, then back so that disp_l always holds the current map
@@ -360,6 +374,90 @@ bool is_pinned(const void* p) {
     return at.type == cudaMemoryTypeHost || at.type == cudaMemoryTypeManaged;
 }
 
+// ---- side outputs ----
+bool aux_wanted(const adc_aux_outputs* a) { return a && (a->origin || a->cost_best || a->cost_second || a->disp_right); }
+bool aux_needs_scratch(const adc_aux_outputs* a) { return a->origin || a->cost_best || a->cost_second; }
+
+// The four outputs of an adc_aux_outputs as (buffer, bytes per pixel), in declaration order.
+struct AuxOut { char* p; size_t el; };
+void aux_outs(const adc_aux_outputs& a, AuxOut o[4]) {
+    o[0] = {reinterpret_cast<char*>(a.origin), 1};
+    o[1] = {reinterpret_cast<char*>(a.cost_best), 4};
+    o[2] = {reinterpret_cast<char*>(a.cost_second), 4};
+    o[3] = {reinterpret_cast<char*>(a.disp_right), 4};
+}
+
+// Device scratch of every lane (when the request needs more than disp_right) and pinned staging of the first
+// `staging_lanes` lanes, allocated once, on the first call that needs them.  A failed allocation leaves the engine as it
+// was, apart from what was already allocated (kept for the next call, freed by adc_destroy).
+int ensure_aux(adc_engine* e, bool scratch, int staging_lanes) {
+    const size_t SN = (size_t)e->S * e->P.dm.N;
+    for (size_t li = 0; li < e->lanes.size(); li++) {
+        Lane& ln = e->lanes[li];
+        if (scratch && !ln.aux_arena) {
+            Carver sz(nullptr);
+            sz.take<uint8_t>(SN); sz.take<uint8_t>(SN); sz.take<float>(SN); sz.take<float>(SN);
+            void* p = nullptr;
+            if (cudaMalloc(&p, sz.off) != cudaSuccess) {
+                cudaGetLastError();
+                return fail(ADC_ERR_NOMEM, "side-output scratch of %zu bytes", sz.off);
+            }
+            Carver c(p);
+            ln.aux.origin = c.take<uint8_t>(SN);
+            ln.aux.lab0 = c.take<uint8_t>(SN);
+            ln.aux.cost_best = c.take<float>(SN);
+            ln.aux.cost_second = c.take<float>(SN);
+            ln.aux_arena = p;
+        }
+        if ((int)li < staging_lanes && !ln.aux_pin) {
+            Carver sz(nullptr);
+            sz.take<uint8_t>(SN); sz.take<float>(SN); sz.take<float>(SN); sz.take<float>(SN);
+            void* p = nullptr;
+            if (cudaHostAlloc(&p, sz.off, cudaHostAllocDefault) != cudaSuccess) {
+                cudaGetLastError();
+                return fail(ADC_ERR_NOMEM, "pinned side-output staging of %zu bytes", sz.off);
+            }
+            Carver c(p);
+            ln.pin_aux.origin = c.take<uint8_t>(SN);
+            ln.pin_aux.cost_best = c.take<float>(SN);
+            ln.pin_aux.cost_second = c.take<float>(SN);
+            ln.pin_aux.disp_right = c.take<float>(SN);
+            ln.aux_pin = p;
+        }
+    }
+    return ADC_OK;
+}
+
+// The lane's device buffers for what `a` asks for (NULL members where it asks for nothing).
+AdcAux wave_aux(const Lane& ln, const adc_aux_outputs& a) {
+    AdcAux x{};
+    if (a.origin) { x.origin = ln.aux.origin; x.lab0 = ln.aux.lab0; }
+    if (a.cost_best) x.cost_best = ln.aux.cost_best;
+    if (a.cost_second) x.cost_second = ln.aux.cost_second;
+    return x;
+}
+
+// Enqueues the copies of the side outputs of nS pairs from the lane's wave into dst (pair `first` of the caller's arrays).
+int copy_aux_out(const Lane& ln, const AdcAux& x, const adc_aux_outputs& dst, size_t first, int nS, size_t N,
+                 cudaMemcpyKind kind, cudaStream_t st) {
+    const void* src[4] = {x.origin, x.cost_best, x.cost_second, ln.w.disp_r};
+    AuxOut o[4];
+    aux_outs(dst, o);
+    for (int k = 0; k < 4; k++)
+        if (o[k].p) CK(cudaMemcpyAsync(o[k].p + first * N * o[k].el, src[k], (size_t)nS * N * o[k].el, kind, st));
+    return ADC_OK;
+}
+
+// The lane's pinned staging for the members `want` asks for (NULL members elsewhere).
+adc_aux_outputs staging_for(const Lane& ln, const adc_aux_outputs& want) {
+    adc_aux_outputs s{};
+    if (want.origin) s.origin = ln.pin_aux.origin;
+    if (want.cost_best) s.cost_best = ln.pin_aux.cost_best;
+    if (want.cost_second) s.cost_second = ln.pin_aux.cost_second;
+    if (want.disp_right) s.disp_right = ln.pin_aux.disp_right;
+    return s;
+}
+
 int drain_lane(adc_engine* e, Lane& ln) {
     if (ln.drain_n == 0) return ADC_OK;
     CK(cudaEventSynchronize(ln.ev_done));
@@ -368,6 +466,12 @@ int drain_lane(adc_engine* e, Lane& ln) {
         float* dst = ln.drain_ptrs ? ln.drain_ptrs[ln.drain_first + i] : ln.drain_base + (size_t)(ln.drain_first + i) * N;
         memcpy(dst, ln.pin_out + (size_t)i * N, N * sizeof(float));
     }
+    AuxOut o[4], s[4];
+    aux_outs(ln.drain_aux, o);
+    aux_outs(ln.pin_aux, s);
+    for (int k = 0; k < 4; k++)
+        if (o[k].p) memcpy(o[k].p + (size_t)ln.drain_first * N * o[k].el, s[k].p, (size_t)ln.drain_n * N * o[k].el);
+    ln.drain_aux = adc_aux_outputs{};
     ln.drain_n = 0;
     return ADC_OK;
 }
@@ -379,7 +483,7 @@ enum SrcKind { SRC_HOST_PTRS, SRC_HOST_STRIDED, SRC_DEVICE_STRIDED };
 // engine's pipelined setting (adc_set_pipelined only changes the asynchronous entry points).
 int run_batch(adc_engine* e, int n, SrcKind kind, const uint8_t* const* lp, const uint8_t* const* rp,
               float* const* dp, const uint8_t* ls, const uint8_t* rs, float* ds, cudaStream_t user, bool pinned,
-              bool force_join = false) {
+              bool force_join = false, const adc_aux_outputs* ua = nullptr) {
     const size_t N = (size_t)e->P.dm.N, IMG = N * 3;
     const int S = e->S, nl = (int)e->lanes.size();
     CK(cudaEventRecord(e->ev_fork, user));
@@ -419,20 +523,27 @@ int run_batch(adc_engine* e, int n, SrcKind kind, const uint8_t* const* lp, cons
         }
         // ---- compute
         cudaStream_t rst = ln.st;   // stream on which the map becomes available
-        int rc = enqueue_pipeline(e, ln, nS, ADC_STAGE_MEDIAN, nullptr);
+        const AdcAux ax = ua ? wave_aux(ln, *ua) : AdcAux{};
+        int rc = enqueue_pipeline(e, ln, nS, ADC_STAGE_MEDIAN, nullptr, ua ? &ax : nullptr);
         if (rc) return rc;
         // ---- outputs
         if (kind == SRC_DEVICE_STRIDED) {
             CK(cudaMemcpyAsync(ds + (size_t)first * N, io.disp_l, (size_t)nS * N * sizeof(float), cudaMemcpyDeviceToDevice, rst));
+            if (ua && (rc = copy_aux_out(ln, ax, *ua, first, nS, N, cudaMemcpyDeviceToDevice, rst))) return rc;
         } else if (pinned) {
             if (kind == SRC_HOST_STRIDED) {
                 CK(cudaMemcpyAsync(ds + (size_t)first * N, io.disp_l, (size_t)nS * N * sizeof(float), cudaMemcpyDeviceToHost, rst));
+                if (ua && (rc = copy_aux_out(ln, ax, *ua, first, nS, N, cudaMemcpyDeviceToHost, rst))) return rc;
             } else {
                 for (int i = 0; i < nS; i++)
                     CK(cudaMemcpyAsync(dp[first + i], io.disp_l + (size_t)i * N, N * sizeof(float), cudaMemcpyDeviceToHost, rst));
             }
         } else {
             CK(cudaMemcpyAsync(ln.pin_out, io.disp_l, (size_t)nS * N * sizeof(float), cudaMemcpyDeviceToHost, rst));
+            if (ua) {
+                if ((rc = copy_aux_out(ln, ax, staging_for(ln, *ua), 0, nS, N, cudaMemcpyDeviceToHost, rst))) return rc;
+                ln.drain_aux = *ua;
+            }
             ln.drain_n = nS; ln.drain_first = first;
             ln.drain_ptrs = kind == SRC_HOST_PTRS ? dp : nullptr;
             ln.drain_base = ds;
@@ -479,6 +590,8 @@ void adc_destroy(adc_engine* e) {
         if (ln.arena) cudaFree(ln.arena);
         if (ln.pin_in) cudaFreeHost(ln.pin_in);
         if (ln.pin_out) cudaFreeHost(ln.pin_out);
+        if (ln.aux_arena) cudaFree(ln.aux_arena);
+        if (ln.aux_pin) cudaFreeHost(ln.aux_pin);
         if (ln.ev_done) cudaEventDestroy(ln.ev_done);
         if (ln.ev_in_free) cudaEventDestroy(ln.ev_in_free);
         if (ln.st) cudaStreamDestroy(ln.st);
@@ -587,27 +700,57 @@ int adc_create(int32_t width, int32_t height, const adc_option* opt, const adc_c
     return ADC_OK;
 }
 
-int adc_match(adc_engine* e, const uint8_t* img_left, const uint8_t* img_right, float* disp_left) {
-    if (!e) return fail(ADC_ERR_ARG, "adc_match: engine is NULL (Match before Initialize)");
-    if (!img_left || !img_right || !disp_left) return fail(ADC_ERR_ARG, "adc_match: NULL image or output pointer");
+}  // extern "C"
+
+namespace {
+
+// One pair on lane 0 through pinned staging: adc_match, and adc_match_aux with `ua` = the wanted side outputs.
+int match_one(adc_engine* e, const uint8_t* img_left, const uint8_t* img_right, float* disp_left, const adc_aux_outputs* ua) {
     CK(cudaSetDevice(e->cfg.device));
     Lane& ln = e->lanes[0];
     const size_t N = (size_t)e->P.dm.N, IMG = N * 3;
-    int rc = drain_lane(e, ln);
+    int rc = ua ? ensure_aux(e, aux_needs_scratch(ua), 1) : ADC_OK;
     if (rc) return rc;
+    if ((rc = drain_lane(e, ln))) return rc;
     CK(cudaStreamSynchronize(ln.st));
     memcpy(ln.pin_in, img_left, IMG);
     memcpy(ln.pin_in + IMG, img_right, IMG);
     CK(cudaEventRecord(e->ev_stage[0], ln.st));
     CK(cudaMemcpyAsync(ln.w.bgr, ln.pin_in, 2 * IMG, cudaMemcpyHostToDevice, ln.st));
-    rc = enqueue_pipeline(e, ln, 1, ADC_STAGE_MEDIAN, e->ev_stage);
+    const AdcAux ax = ua ? wave_aux(ln, *ua) : AdcAux{};
+    rc = enqueue_pipeline(e, ln, 1, ADC_STAGE_MEDIAN, e->ev_stage, ua ? &ax : nullptr);
     if (rc) return rc;
     CK(cudaMemcpyAsync(ln.pin_out, ln.w.disp_l, N * sizeof(float), cudaMemcpyDeviceToHost, ln.st));
+    if (ua && (rc = copy_aux_out(ln, ax, staging_for(ln, *ua), 0, 1, N, cudaMemcpyDeviceToHost, ln.st))) return rc;
     CK(cudaEventRecord(e->ev_stage[6], ln.st));
     CK(cudaStreamSynchronize(ln.st));
     memcpy(disp_left, ln.pin_out, N * sizeof(float));
+    if (ua) {
+        AuxOut o[4], s[4];
+        aux_outs(*ua, o);
+        aux_outs(ln.pin_aux, s);
+        for (int k = 0; k < 4; k++)
+            if (o[k].p) memcpy(o[k].p, s[k].p, N * o[k].el);
+    }
     for (int i = 0; i < 6; i++) CK(cudaEventElapsedTime(&e->stage_ms[i], e->ev_stage[i], e->ev_stage[i + 1]));
     return ADC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int adc_match(adc_engine* e, const uint8_t* img_left, const uint8_t* img_right, float* disp_left) {
+    if (!e) return fail(ADC_ERR_ARG, "adc_match: engine is NULL (Match before Initialize)");
+    if (!img_left || !img_right || !disp_left) return fail(ADC_ERR_ARG, "adc_match: NULL image or output pointer");
+    return match_one(e, img_left, img_right, disp_left, nullptr);
+}
+
+int adc_match_aux(adc_engine* e, const uint8_t* img_left, const uint8_t* img_right, float* disp_left,
+                  const adc_aux_outputs* aux) {
+    if (!e) return fail(ADC_ERR_ARG, "adc_match_aux: engine is NULL (Match before Initialize)");
+    if (!img_left || !img_right || !disp_left) return fail(ADC_ERR_ARG, "adc_match_aux: NULL image or output pointer");
+    return match_one(e, img_left, img_right, disp_left, aux_wanted(aux) ? aux : nullptr);
 }
 
 int adc_get_right_disparity(adc_engine* e, float* disp_right) {
@@ -648,6 +791,27 @@ int adc_match_batch_strided(adc_engine* e, int32_t n, const uint8_t* left, const
     return ADC_OK;
 }
 
+int adc_match_batch_strided_aux(adc_engine* e, int32_t n, const uint8_t* left, const uint8_t* right, float* disp,
+                                const adc_aux_outputs* aux) {
+    if (!e) return fail(ADC_ERR_ARG, "adc_match_batch_strided_aux: engine is NULL");
+    if (n < 0 || (n > 0 && (!left || !right || !disp))) return fail(ADC_ERR_ARG, "adc_match_batch_strided_aux: bad arguments");
+    if (n == 0) return ADC_OK;
+    const adc_aux_outputs* ua = aux_wanted(aux) ? aux : nullptr;
+    CK(cudaSetDevice(e->cfg.device));
+    bool pinned = is_pinned(left) && is_pinned(right) && is_pinned(disp);
+    if (ua) {
+        AuxOut o[4];
+        aux_outs(*ua, o);
+        for (int k = 0; k < 4; k++) pinned = pinned && (!o[k].p || is_pinned(o[k].p));
+        int rc = ensure_aux(e, aux_needs_scratch(ua), pinned ? 0 : (int)e->lanes.size());
+        if (rc) return rc;
+    }
+    int rc = run_batch(e, n, SRC_HOST_STRIDED, nullptr, nullptr, nullptr, left, right, disp, e->main_st, pinned, true, ua);
+    if (rc) return rc;
+    CK(cudaStreamSynchronize(e->main_st));
+    return ADC_OK;
+}
+
 int adc_match_batch_pinned_async(adc_engine* e, int32_t n, const uint8_t* left, const uint8_t* right, float* disp, void* stream) {
     if (!e) return fail(ADC_ERR_ARG, "adc_match_batch_pinned_async: engine is NULL");
     if (n < 0 || (n > 0 && (!left || !right || !disp))) return fail(ADC_ERR_ARG, "adc_match_batch_pinned_async: bad arguments");
@@ -664,6 +828,21 @@ int adc_match_batch_device(adc_engine* e, int32_t n, const uint8_t* d_left, cons
     if (n == 0) return ADC_OK;
     CK(cudaSetDevice(e->cfg.device));
     return run_batch(e, n, SRC_DEVICE_STRIDED, nullptr, nullptr, nullptr, d_left, d_right, d_disp, (cudaStream_t)stream, true);
+}
+
+int adc_match_batch_device_aux(adc_engine* e, int32_t n, const uint8_t* d_left, const uint8_t* d_right, float* d_disp,
+                               const adc_aux_outputs* aux, void* stream) {
+    if (!e) return fail(ADC_ERR_ARG, "adc_match_batch_device_aux: engine is NULL");
+    if (n < 0 || (n > 0 && (!d_left || !d_right || !d_disp))) return fail(ADC_ERR_ARG, "adc_match_batch_device_aux: bad arguments");
+    if (n == 0) return ADC_OK;
+    const adc_aux_outputs* ua = aux_wanted(aux) ? aux : nullptr;
+    CK(cudaSetDevice(e->cfg.device));
+    if (ua) {
+        int rc = ensure_aux(e, aux_needs_scratch(ua), 0);
+        if (rc) return rc;
+    }
+    return run_batch(e, n, SRC_DEVICE_STRIDED, nullptr, nullptr, nullptr, d_left, d_right, d_disp, (cudaStream_t)stream, true,
+                     false, ua);
 }
 
 void* adc_host_alloc(size_t bytes) {
@@ -790,6 +969,14 @@ int adc_profile_kernel(adc_engine* e, int32_t kernel_id, int32_t reps, float* av
             case 7: if (!adc_launch_arm_sum2(P, w, w.volA, w.volB, 0, w.sup_v, ln.st, &e->launches)) return fail(ADC_ERR_UNSUPPORTED, "fused horizontal arm sums not applicable"); bytes = 2 * V + 6 * N; break;
             case 8: adc_launch_arm_sum(P, w, w.volA, w.volB, 0, w.sup_v, ln.st, &e->launches); bytes = 2 * V + 6 * N; break;
             case 9: adc_launch_arm_sum(P, w, w.volA, w.volB, 1, nullptr, ln.st, &e->launches); bytes = 2 * V + 4 * N; break;
+            case 10: {
+                int rc = ensure_aux(e, true, 0);
+                if (rc) return rc;
+                const AdcAux ax{ln.aux.origin, nullptr, ln.aux.cost_best, ln.aux.cost_second};
+                if (adc_launch_wta_aux(P, w, w.volA, ax, ln.st, &e->launches)) return fail(ADC_ERR_UNSUPPORTED, "wta");
+                bytes = V + 17 * N;
+                break;
+            }
             default: return fail(ADC_ERR_ARG, "adc_profile_kernel: unknown kernel id %d", kernel_id);
         }
     }

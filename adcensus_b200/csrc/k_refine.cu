@@ -7,6 +7,7 @@
 // answer.  Each kernel below is a parallel schedule that provably reproduces the sequential
 // result (argument given at each kernel); none of them approximates.
 #include "adc_common.cuh"
+#include "../../include/adcensus_b200.h"
 #include <stdlib.h>
 #include <algorithm>
 
@@ -834,6 +835,28 @@ void adc_launch_interp_list(const AdcParams& P, const AdcWave& w, int k, cudaStr
         return;
     }
     k_interpolate<<<grid, 256, 0, st>>>(P, k, w.bgr, w.disp_l, w.disp_t, w.pend, w.counters, w.ray_sin, w.ray_cos, w.ray_off);
+    ++*launches;
+}
+
+// Origin map (side output, adcensus_b200.h ADC_ORIGIN_*), after the last filling step that ran.  Every voting kernel
+// clears the label of a pixel it fills and interpolation leaves the labels alone, so: a pixel listed before voting
+// (lab0) and no longer listed after it was filled by voting; one still listed and now finite, by interpolation.  Without
+// filling the labels never change, and every listed pixel is still Invalid_Float.  origin holds the WTA-invalid flag.
+__global__ void k_origin(AdcDims dm, const uint8_t* __restrict__ lab0, const uint8_t* __restrict__ lab1,
+                         const float* __restrict__ disp, uint8_t* __restrict__ origin) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= dm.N) return;
+    const size_t o = (size_t)blockIdx.y * dm.N + i;
+    const uint8_t l0 = lab0[o];
+    uint8_t code = ADC_ORIGIN_MATCHED;
+    if (disp[o] == ADC_INVALID_F) code = ADC_ORIGIN_INVALID;
+    else if (l0 != 0) code = lab1[o] == 0 ? l0 : (uint8_t)(l0 + 2);   // 1, 2: voted mismatch / occlusion; 3, 4: interpolated
+    origin[o] |= code;
+}
+
+void adc_launch_origin(const AdcParams& P, const AdcWave& w, const AdcAux& aux, cudaStream_t st, unsigned long long* launches) {
+    dim3 grid((P.dm.N + 255) / 256, w.S);
+    k_origin<<<grid, 256, 0, st>>>(P.dm, aux.lab0, w.label, w.disp_l, aux.origin);
     ++*launches;
 }
 

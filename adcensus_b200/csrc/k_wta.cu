@@ -1,6 +1,7 @@
 // k_wta.cu -- stage 4: winner-takes-all with parabola refinement for the left view and, from the
 // same volume, for the right view (reference: ADCensusStereo.cpp:188-243 and :245-310).
 #include "adc_common.cuh"
+#include "../../include/adcensus_b200.h"
 
 // Parabola through (best-1, best, best+1), ADCensusStereo.cpp:234-240.  Explicit _rn intrinsics keep
 // nvcc from contracting c1 + c2 - 2*min into an FMA.
@@ -36,8 +37,24 @@ __device__ __forceinline__ float adc_subpixel(float c1, float c2, float cmin, in
 #define WT_RS (WT_PX + 3)      // row stride of the right tile: the skewed stores of a warp (columns cj .. cj + 7, four quads) land in 32
                                // different banks: bank = cj + 8 kq + const (with stride 128 it is cj - 4 kq: pairs of lanes collide)
 
-__global__ void __launch_bounds__(WT_PX, 6)
-k_wta(AdcDims dm, const float* __restrict__ vol, float* __restrict__ disp_l, float* __restrict__ disp_r) {
+// Side outputs (AUX = true): the cost of the left winner b and the least cost two or more disparities away from it come
+// out of the same ascending scan with O(1) state, carried across chunks like (minimum, argmin):
+//   pre  min over the indices <= i - 2, fed through the one-step delay q1
+//   a strict new minimum at i:   b = i, sec = pre      (everything seen so far that is at least two below i)
+//   otherwise, when i >= b + 2:  sec = min(sec, a)     (i = b + 1 is skipped)
+// th is b + 2 relative to the chunk, so that the test is one compare against the unrolled chunk index.
+struct WtaSecond { float pre, q1, sec; int th; };
+__device__ __forceinline__ void wta_second(WtaSecond& s, bool newmin, float a, int k) {
+    if (newmin) { s.sec = s.pre; s.th = k + 2; }
+    else if (k >= s.th) s.sec = a < s.sec ? a : s.sec;
+    s.pre = s.q1 < s.pre ? s.q1 : s.pre;
+    s.q1 = a;
+}
+
+// AUX = false is the plain kernel; AUX = true keeps one CTA fewer per SM for the four extra registers of the state above
+template <bool AUX>
+__global__ void __launch_bounds__(WT_PX, AUX ? 5 : 6)
+k_wta(AdcDims dm, const float* __restrict__ vol, float* __restrict__ disp_l, float* __restrict__ disp_r, AdcAux aux) {
     __shared__ __align__(16) float tl[WT_PX * WT_LS];
     __shared__ float tr[WT_DC * WT_RS];
     const int pair = blockIdx.z, y = blockIdx.y, x0 = blockIdx.x * WT_PX;
@@ -48,6 +65,7 @@ k_wta(AdcDims dm, const float* __restrict__ vol, float* __restrict__ disp_l, flo
     const float4 LARGE4 = make_float4(ADC_LARGE_F, ADC_LARGE_F, ADC_LARGE_F, ADC_LARGE_F);
     float lbest = ADC_LARGE_F, rbest = ADC_LARGE_F;     // min_cost starts at Large_Float (:209, :266)
     int lbd = -1, rbd = -1;                             // argmin as index d - dmin, -1 = none yet
+    WtaSecond s2{ADC_INVALID_F, ADC_INVALID_F, ADC_INVALID_F, 1};
     float4 vl[WT_PX / 32], vr[WT_RT];
     // The loads of chunk c + 1 are issued before chunk c is scanned and land in registers while the scan runs.
     auto fetch = [&](int d0) {
@@ -97,19 +115,24 @@ k_wta(AdcDims dm, const float* __restrict__ vol, float* __restrict__ disp_l, flo
 #pragma unroll
                 for (int j = 0; j < 4; j++) {
                     const float b = pr[(k4 + j) * WT_RS];
-                    if (lbest > a[j]) { lbest = a[j]; lk = k4 + j; }
+                    const bool nl = lbest > a[j];
+                    if (nl) { lbest = a[j]; lk = k4 + j; }
+                    if (AUX) wta_second(s2, nl, a[j], k4 + j);
                     if (rbest > b) { rbest = b; rk = k4 + j; }
                 }
             }
         } else {
             for (int k = 0; k < dn; k++) {
                 const float a = pl[k ^ sw], b = pr[k * WT_RS];
-                if (lbest > a) { lbest = a; lk = k; }
+                const bool nl = lbest > a;
+                if (nl) { lbest = a; lk = k; }
+                if (AUX) wta_second(s2, nl, a, k);
                 if (rbest > b) { rbest = b; rk = k; }
             }
         }
         if (lk >= 0) lbd = d0 + lk;
         if (rk >= 0) rbd = d0 + rk;
+        if (AUX) s2.th -= WT_DC;
         __syncthreads();
     }
     const int x = x0 + t;
@@ -122,6 +145,11 @@ k_wta(AdcDims dm, const float* __restrict__ vol, float* __restrict__ disp_l, flo
             out = adc_subpixel(__ldg(v - 1), __ldg(v + 1), lbest, dm.dmin + lbd);
         }
         disp_l[o] = out;
+        if (AUX) {
+            if (aux.cost_best) aux.cost_best[o] = lbest;
+            if (aux.cost_second) aux.cost_second[o] = s2.sec;
+            if (aux.origin) aux.origin[o] = out == ADC_INVALID_F ? ADC_ORIGIN_WTA_INVALID : 0;
+        }
     }
     {   // right view: a minimum at either end gives the integer disparity, not Invalid (:290-293); `best` starts at 0
         // (not dmin) when no column was valid, as in the reference (:271); a parabola neighbour whose column lies
@@ -143,7 +171,15 @@ k_wta(AdcDims dm, const float* __restrict__ vol, float* __restrict__ disp_l, flo
 
 int adc_launch_wta(const AdcParams& P, const AdcWave& w, const float* vol, cudaStream_t st, unsigned long long* launches) {
     dim3 grid((P.dm.W + WT_PX - 1) / WT_PX, P.dm.H, w.S);
-    k_wta<<<grid, WT_PX, 0, st>>>(P.dm, vol, w.disp_l, w.disp_r);
+    k_wta<false><<<grid, WT_PX, 0, st>>>(P.dm, vol, w.disp_l, w.disp_r, AdcAux{});
+    ++*launches;
+    return 0;
+}
+
+int adc_launch_wta_aux(const AdcParams& P, const AdcWave& w, const float* vol, const AdcAux& aux, cudaStream_t st,
+                       unsigned long long* launches) {
+    dim3 grid((P.dm.W + WT_PX - 1) / WT_PX, P.dm.H, w.S);
+    k_wta<true><<<grid, WT_PX, 0, st>>>(P.dm, vol, w.disp_l, w.disp_r, aux);
     ++*launches;
     return 0;
 }

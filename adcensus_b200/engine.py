@@ -60,6 +60,22 @@ MAX_DISPARITY_RANGE, MAX_DISPARITY_RANGE_WIDE = 256, 512
 DBG_NO_RAY_TABLE, DBG_VOTE_ENUM, DBG_VOTE_GLOBAL_STATE, DBG_UNFUSED_AGG = 1, 2, 4, 8
 
 
+class AuxOutputs(ctypes.Structure):
+    """Mirror of adc_aux_outputs: device or host pointers of the side outputs, 0 / None = not wanted."""
+    _fields_ = [("origin", ctypes.c_void_p), ("cost_best", ctypes.c_void_p), ("cost_second", ctypes.c_void_p),
+                ("disp_right", ctypes.c_void_p)]
+
+
+assert ctypes.sizeof(AuxOutputs) == 32
+
+# adc_aux_outputs.origin: how a pixel's value was obtained (before discontinuity adjustment and the median filter)
+ADC_ORIGIN_MATCHED, ADC_ORIGIN_VOTED_MISMATCH, ADC_ORIGIN_VOTED_OCCLUSION = 0, 1, 2
+ADC_ORIGIN_INTERP_MISMATCH, ADC_ORIGIN_INTERP_OCCLUSION, ADC_ORIGIN_INVALID = 3, 4, 5
+ADC_ORIGIN_WTA_INVALID = 8   # flag OR-ed onto the code: WTA itself returned Invalid_Float
+AUX_NAMES = ("origin", "cost_best", "cost_second", "disp_right")
+_AUX_DTYPE = {"origin": np.uint8, "cost_best": np.float32, "cost_second": np.float32, "disp_right": np.float32}
+
+
 class AdcError(RuntimeError):
     pass
 
@@ -93,6 +109,10 @@ def load_library() -> ctypes.CDLL:
     L.adc_match_batch_strided.argtypes = [vp, i32, u8p, u8p, f32p]
     L.adc_match_batch_device.argtypes = [vp, i32, u8p, u8p, f32p, vp]
     L.adc_match_batch_pinned_async.argtypes = [vp, i32, u8p, u8p, f32p, vp]
+    auxp = ctypes.POINTER(AuxOutputs)
+    L.adc_match_aux.argtypes = [vp, u8p, u8p, f32p, auxp]
+    L.adc_match_batch_strided_aux.argtypes = [vp, i32, u8p, u8p, f32p, auxp]
+    L.adc_match_batch_device_aux.argtypes = [vp, i32, u8p, u8p, f32p, auxp, vp]
     L.adc_host_alloc.argtypes = [ctypes.c_size_t]
     L.adc_host_alloc.restype = vp
     L.adc_host_free.argtypes = [vp]
@@ -186,6 +206,41 @@ class Engine:
         _check(self._L.adc_match_batch_strided(self._h, n, lefts.ctypes.data, rights.ctypes.data, disp.ctypes.data))
         return disp
 
+    def _aux_arrays(self, want, lead=()):
+        unknown = set(want) - set(AUX_NAMES)
+        if unknown:
+            raise ValueError(f"unknown side outputs {sorted(unknown)}; choose from {AUX_NAMES}")
+        out = {k: np.empty(lead + (self.height, self.width), _AUX_DTYPE[k]) for k in AUX_NAMES if k in want}
+        return out, AuxOutputs(**{k: a.ctypes.data for k, a in out.items()})
+
+    def match_aux(self, left, right, want=AUX_NAMES):
+        """match() with side outputs: (disp, {name: [H][W] array}) for the names in `want` (AUX_NAMES)."""
+        left = _img(left, (self.height, self.width, 3))
+        right = _img(right, (self.height, self.width, 3))
+        disp = np.empty((self.height, self.width), np.float32)
+        out, aux = self._aux_arrays(want)
+        _check(self._L.adc_match_aux(self._h, left.ctypes.data, right.ctypes.data, disp.ctypes.data, ctypes.byref(aux)))
+        return disp, out
+
+    def match_batch_aux(self, lefts, rights, want=AUX_NAMES):
+        """match_batch() with side outputs: (disp [n][H][W], {name: [n][H][W] array})."""
+        lefts = np.ascontiguousarray(lefts, np.uint8)
+        rights = np.ascontiguousarray(rights, np.uint8)
+        n = lefts.shape[0]
+        if lefts.shape != (n, self.height, self.width, 3) or rights.shape != lefts.shape:
+            raise ValueError("expected [n][H][W][3] uint8 arrays")
+        disp = np.empty((n, self.height, self.width), np.float32)
+        out, aux = self._aux_arrays(want, (n,))
+        _check(self._L.adc_match_batch_strided_aux(self._h, n, lefts.ctypes.data, rights.ctypes.data, disp.ctypes.data,
+                                                   ctypes.byref(aux)))
+        return disp, out
+
+    def match_batch_device_aux(self, n: int, d_left: int, d_right: int, d_disp: int, origin: int = 0, cost_best: int = 0,
+                               cost_second: int = 0, disp_right: int = 0, stream: int = 0):
+        """match_batch_device() with side outputs into device buffers (ints, 0 = not wanted), [n][H][W] each."""
+        aux = AuxOutputs(origin or None, cost_best or None, cost_second or None, disp_right or None)
+        _check(self._L.adc_match_batch_device_aux(self._h, n, d_left, d_right, d_disp, ctypes.byref(aux), stream))
+
     def match_batch_ptrs(self, lefts, rights):
         """Pointer-array form (adc_match_batch): independent per-pair buffers."""
         n = len(lefts)
@@ -217,7 +272,7 @@ class Engine:
         return list(out)
 
     PROFILE_KERNELS = {"cost_volume": 0, "arm_sum_h": 1, "arm_sum_v_div": 2, "scanline_x": 3, "scanline_y": 4, "wta": 5,
-                       "arm_sum2_v": 6, "arm_sum2_h": 7, "arm_sum_h_div": 8, "arm_sum_v": 9}
+                       "arm_sum2_v": 6, "arm_sum2_h": 7, "arm_sum_h_div": 8, "arm_sum_v": 9, "wta_aux": 10}
 
     def profile_kernel(self, name: str, reps: int = 5):
         """(mean ms per launch over one wave, algorithmic bytes per launch) of one pipeline kernel."""
@@ -312,6 +367,14 @@ class ADCensusStereo:
             np.copyto(disp_left.reshape(out.shape), out)
             return True
         return out
+
+    def MatchWithConfidence(self, img_left, img_right):
+        """Extension (not in the reference): (disp, origin, cost_best, cost_second) of one pair, see Engine.match_aux;
+        False where Match returns False."""
+        if self._engine is None or img_left is None or img_right is None:
+            return False
+        disp, aux = self._engine.match_aux(img_left, img_right, ("origin", "cost_best", "cost_second"))
+        return disp, aux["origin"], aux["cost_best"], aux["cost_second"]
 
     def Reset(self, width: int, height: int, option: ADCensusOption) -> bool:
         self.Release()

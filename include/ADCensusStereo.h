@@ -43,6 +43,11 @@ public:
     bool Initialize(const sint32& width, const sint32& height, const ADCensusOption& option, sint32 max_disparity_range);
     // n independent pairs in one call: left/right [n][H][W][3], disp [n][H][W] (host memory).
     bool MatchBatch(sint32 n, const uint8* left, const uint8* right, float32* disp);
+    // Match plus per-pixel confidence (adc_match_aux): origin = ADC_ORIGIN_* code of each pixel (measured, voted,
+    // interpolated, invalid), cost_best / cost_second = the winner's aggregated cost and the least cost two or more
+    // disparities away from it.  width*height each; any of the three may be null.  Prints the timing lines Match prints.
+    bool MatchWithConfidence(const uint8* img_left, const uint8* img_right, float32* disp_left, uint8* origin,
+                             float32* cost_best, float32* cost_second);
     adc_engine* handle() const { return engine_; }
 
 private:

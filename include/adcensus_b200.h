@@ -103,8 +103,42 @@ int adc_match(adc_engine* e, const uint8_t* img_left, const uint8_t* img_right, 
 /* The right-view disparity map of the most recent adc_match call: what the reference computes into its private
  * disp_right_ (ADCensusStereo::ComputeDisparityRight, ADCensusStereo.cpp:245-310) for the left-right check and never
  * hands out -- float32 [H][W], sub-pixel, not refined (a minimum at either end of the range is the integer disparity).
- * Host pointer.  SURVEY.md 8(f) rank 4. */
+ * Host pointer.  SURVEY.md 8(f) rank 4.  Batch callers get the same map per pair through adc_aux_outputs.disp_right of
+ * adc_match_batch_strided_aux / adc_match_batch_device_aux. */
 int adc_get_right_disparity(adc_engine* e, float* disp_right);
+
+/* ---- side outputs (confidence) ----------------------------------------------------------------
+ * Per pair, [H][W], left view, of the same run as the map they come with:
+ *   origin       how the pixel's value was obtained, before discontinuity adjustment and the median filter (those two
+ *                stages touch every pixel and do not change it): one ADC_ORIGIN_* code, with ADC_ORIGIN_WTA_INVALID
+ *                OR-ed on where WTA itself returned Invalid_Float (the minimum lay at an end of the disparity range).
+ *   cost_best    min over d in [0, D) of the aggregated cost WTA scans (the output of the fourth scanline pass): the
+ *                cost of the WTA winner b (the first minimum in ascending d).
+ *   cost_second  min of that cost over the d with |d - b| >= 2; +inf where there is none (range < 3, or range 3 with
+ *                b = 1).  cost_best / cost_second is the usual peak-ratio confidence.
+ *   disp_right   the right-view map, exactly what adc_get_right_disparity returns after adc_match of that pair.
+ * Any member may be NULL (not wanted).  aux == NULL, or all four members NULL, runs exactly the plain call. */
+typedef struct adc_aux_outputs {
+    uint8_t* origin;      /* [n][H][W] ADC_ORIGIN_* */
+    float*   cost_best;   /* [n][H][W] */
+    float*   cost_second; /* [n][H][W] */
+    float*   disp_right;  /* [n][H][W] */
+} adc_aux_outputs;
+
+enum {
+    ADC_ORIGIN_MATCHED = 0,            /* a WTA value that passed the left-right check (any finite WTA value without it) */
+    ADC_ORIGIN_VOTED_MISMATCH = 1,     /* in the mismatch list after the outlier stage, filled by region voting */
+    ADC_ORIGIN_VOTED_OCCLUSION = 2,    /* in the occlusion list after the outlier stage, filled by region voting */
+    ADC_ORIGIN_INTERP_MISMATCH = 3,    /* still in the mismatch list after voting, filled by proper interpolation */
+    ADC_ORIGIN_INTERP_OCCLUSION = 4,   /* still in the occlusion list after voting, filled by proper interpolation */
+    ADC_ORIGIN_INVALID = 5,            /* still Invalid_Float after the last filling step that ran */
+    ADC_ORIGIN_WTA_INVALID = 8         /* flag: WTA returned Invalid_Float (minimum at an end of the range) */
+};
+
+/* adc_match with side outputs.  Host pointers, synchronous.  The side outputs' device scratch and pinned staging are
+ * allocated on the first call that asks for them (ADC_ERR_NOMEM if that fails; the engine stays usable). */
+int adc_match_aux(adc_engine* e, const uint8_t* img_left, const uint8_t* img_right, float* disp_left,
+                  const adc_aux_outputs* aux);
 
 /* Batched Match over n independent pairs (the data-parallel form of the call above; the
  * reference would loop Match).  Pointers are host pointers; pinned buffers are copied
@@ -115,6 +149,9 @@ int adc_match_batch(adc_engine* e, int32_t n, const uint8_t* const* img_left,
 
 /* Same, contiguous host arrays: left/right [n][H][W][3], disp [n][H][W]. */
 int adc_match_batch_strided(adc_engine* e, int32_t n, const uint8_t* left, const uint8_t* right, float* disp);
+/* Same, with side outputs (see adc_aux_outputs): host buffers, pageable or pinned, synchronous. */
+int adc_match_batch_strided_aux(adc_engine* e, int32_t n, const uint8_t* left, const uint8_t* right, float* disp,
+                                const adc_aux_outputs* aux);
 
 /* Same, but the arrays already live in device memory (HBM-resident form used for the
  * kernel-only throughput figure).  Work is enqueued on the engine's streams, fork/joined on
@@ -122,6 +159,10 @@ int adc_match_batch_strided(adc_engine* e, int32_t n, const uint8_t* left, const
  * the caller brackets it with its own events. */
 int adc_match_batch_device(adc_engine* e, int32_t n, const uint8_t* d_left, const uint8_t* d_right,
                            float* d_disp, void* stream);
+/* Same, with side outputs (see adc_aux_outputs) in device memory, complete when d_disp is (in pipelined mode: after
+ * adc_join). */
+int adc_match_batch_device_aux(adc_engine* e, int32_t n, const uint8_t* d_left, const uint8_t* d_right,
+                               float* d_disp, const adc_aux_outputs* aux, void* stream);
 
 /* Asynchronous host-buffer form for callers that pipeline their own I/O: buffers must be pinned
  * (adc_host_alloc or cudaHostAlloc / cudaHostRegister).  Enqueues H2D, compute and D2H, joined on
@@ -155,7 +196,8 @@ int adc_get_config(const adc_engine* e, adc_config* out);
  * wave of wave_pairs pairs: kernel_id 0 = cost volume, 1 = horizontal arm sum, 2 = vertical arm sum
  * with division, 3 = scanline pass along x, 4 = scanline pass along y, 5 = WTA left+right, 6 / 7 = the fused
  * vertical / horizontal double pass of the aggregation (divide + sum, intermediate in shared memory), 8 = horizontal
- * arm sum with division, 9 = vertical arm sum without division.
+ * arm sum with division, 9 = vertical arm sum without division, 10 = WTA left+right that also writes the side outputs
+ * cost_best, cost_second and the WTA-invalid flag of the origin map.
  * algorithmic_bytes (optional) receives the bytes one launch must move (SURVEY.md section 8d). */
 int adc_profile_kernel(adc_engine* e, int32_t kernel_id, int32_t reps, float* avg_ms, double* algorithmic_bytes);
 
